@@ -222,7 +222,7 @@ def grpc_h2_main(args):
     pin_to_gpu_numa(dev)
     hbm_peak, peak_src = read_peaks()
     n_conns, K, msg_len = 256, args.frames_per_stream, args.payload if args.payload != 1024 else 4096
-    steps, warmup = max(1, min(args.steps, 200)), max(3, args.warmup)
+    steps, warmup = max(1, args.steps), max(3, args.warmup)
     rng = random.Random(20260921 + rank)
     ctx = brpc_b200.Context(device=dev, max_batch_bytes=64 << 20, max_msgs=1 << 16, max_runs=1024, max_resp_bytes=128 << 20)
     message = bytes(rng.choice(b"abcdefghijklmnopqrstuvwxyz0123456789") for _ in range(msg_len))
@@ -340,7 +340,7 @@ def stream_snappy_main(args):
     dev = local_rank if use_dist else 0
     torch.cuda.set_device(dev)
     hbm_peak, peak_src = read_peaks()
-    steps, warmup = max(1, min(args.steps, 100)), max(3, args.warmup)
+    steps, warmup = max(1, args.steps), max(3, args.warmup)
     RAW = 256 << 10
     rng = np.random.default_rng(20260921 + rank)
     table = np.frombuffer(b"abcdefghijklmnopqrstuvwxyz0123456789ABCDEFGHIJKLMNOPQRSTUVWXYZ", np.uint8)
@@ -506,6 +506,33 @@ def fill_batch_plain(data, run_mib, rank, world, payload=PAYLOAD, checksum=0, ki
     return runs, int(total), N_SOCKETS * stride
 
 
+def dump_outputs(out_dir, rs, msgs, resp, sample=4096, reply_bytes=2048):
+    """What a caller of the timed path receives for the batch, as float64 / float32 .npy files: per connection, run_<field>
+    and the zlib CRC-32s of all its message descriptors (run_msgs_crc32) and of its replies in order (run_reply_crc32); msg_index, a
+    fixed seeded sample of `sample` messages, with msg_<field> their descriptors and reply_bytes / reply_bytes_off the first
+    `reply_bytes` bytes of their replies, concatenated.  Every value is exact: the 64-bit ids rpc_press.cpp writes stay
+    below 2^53."""
+    import zlib
+    os.makedirs(out_dir, exist_ok=True)
+    save = lambda name, a, dt=np.float64: np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a).astype(dt))
+    for f in rs.dtype.names:
+        save("run_" + f, rs[f])
+    resp = np.asarray(resp)
+    save("run_msgs_crc32", [zlib.crc32(msgs[int(r["first_msg"]):int(r["first_msg"]) + int(r["n_msgs"])].tobytes()) for r in rs])
+    offs, lens = msgs["resp_off"].astype(np.int64), msgs["resp_len"].astype(np.int64)
+    crc = np.zeros(len(rs), np.uint32)
+    for r, o, n in zip(msgs["run_idx"], offs, lens):
+        crc[r] = zlib.crc32(resp[o:o + n], int(crc[r]))
+    save("run_reply_crc32", crc)
+    idx = np.sort(np.random.default_rng(20260921).choice(len(msgs), min(sample, len(msgs)), replace=False))
+    save("msg_index", idx)
+    for f in msgs.dtype.names:
+        save("msg_" + f, msgs[f][idx])
+    parts = [resp[o:o + min(n, reply_bytes)] for o, n in zip(offs[idx], lens[idx])]
+    save("reply_bytes", np.concatenate(parts) if parts else np.zeros(0, np.uint8), np.float32)
+    save("reply_bytes_off", np.cumsum([0] + [len(p) for p in parts]))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -521,11 +548,13 @@ def main():
     ap.add_argument("--payload-kind", type=int, default=0, help="0 = 'r' fill, 1 = random over 62 symbols")
     ap.add_argument("--no-latency", action="store_true")
     ap.add_argument("--pipeline", type=int, default=2, help="resident batches in flight per GPU (one ctx + stream each)")
-    ap.add_argument("--min-seconds", type=float, default=1.0, help="the timed region of `value` lasts at least this long: a step repeats the pass")
     ap.add_argument("--workload", default="echo", choices=["echo", "stream_snappy", "grpc_h2"],
                     help="echo = the headline metric; stream_snappy = BASELINE configs[4] (256 KiB snappy streaming frames), grpc_h2 = configs[3]")
     ap.add_argument("--frames-per-stream", type=int, default=8)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed to DIR/<name>.npy (echo workload)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.workload != "echo" or args.impl != "b200"):
+        ap.error("--dump-outputs covers the echo workload of the b200 implementation")
     global N_SOCKETS
     N_SOCKETS = max(1, args.sockets)
     if args.run_mib == int(args.run_mib):
@@ -605,8 +634,7 @@ def main():
 
     # ---- value: resident batches, kernel pipeline only -----------------------------------------
     # `--pipeline D` contexts (own buffers + stream) hold the same batch; passes alternate over them so the latency-bound
-    # front stages of one pass overlap the bandwidth kernel of another.  A STEP is `passes_per_step` passes over the batch:
-    # enough for the timed region to last --min-seconds whatever --steps is, so the clock samples below cover it.
+    # front stages of one pass overlap the bandwidth kernel of another.  A STEP is one pass over the batch.
     depth = max(1, args.pipeline)
     ctxs = [ctx] + [mk() for _ in range(depth - 1)]
     for cx in ctxs:
@@ -615,15 +643,6 @@ def main():
         ctxs[s_ % depth].launch()
     for cx in ctxs:
         cx.wait()
-    t0 = time.perf_counter()
-    for s_ in range(8 * depth):
-        ctxs[s_ % depth].launch()
-    for cx in ctxs:
-        cx.wait()
-    est = (time.perf_counter() - t0) / (8 * depth)
-    ppass = max(1, int(np.ceil(args.min_seconds / max(1e-9, steps * est))))
-    if use_dist:
-        t_pp = torch.tensor([ppass], dtype=torch.int64, device="cuda"); dist.all_reduce(t_pp, op=dist.ReduceOp.MAX); ppass = int(t_pp.item())
     launches_per_pass = ctx.execute()[1]
     fused = ctx.batch_info()["fused"]
     for cx in ctxs:
@@ -631,17 +650,19 @@ def main():
     sampler = ClockSampler(dev); sampler.start()
     barrier()
     t0 = time.perf_counter()
-    for s_ in range(steps * ppass):
+    for s_ in range(steps):
         ctxs[s_ % depth].launch()
     for cx in ctxs:
         cx.wait()
     barrier()
     wall_ms = (time.perf_counter() - t0) * 1e3
-    dev_ms = max(ctxs[0].elapsed_ms_to(cx) for cx in ctxs[:min(depth, steps * ppass)])
-    n_launch = steps * ppass * launches_per_pass
+    dev_ms = max(ctxs[0].elapsed_ms_to(cx) for cx in ctxs[:min(depth, steps)])
+    n_launch = steps * launches_per_pass
     for cx in ctxs[1:]:       # every in-flight copy produced the same, correct result
         r2, m2, p2, _ = cx.download()
         assert len(m2) == n_full and np.array_equal(m2["resp_len"], msgs["resp_len"]) and np.array_equal(m2["status"], msgs["status"])
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *ctxs[(steps - 1) % depth].download()[:3])
     # per-stage device times (CUDA events between the launches of one pass), averaged
     stage_acc = {}
     for _ in range(5):
@@ -769,10 +790,9 @@ def main():
     dev_ms_max, wall_ms_max, e_copy, e_ref, e_pull, e_iov = t_dev.tolist()
     total_msgs = tot.item()
     ms_per_step = dev_ms_max / steps
-    value = total_msgs * ppass / (ms_per_step * 1e-3)
+    value = total_msgs / (ms_per_step * 1e-3)
 
     if rank == 0:
-        config["passes_per_step"] = ppass
         config["value_path"] = "k_fused (decode + echo + pack in one pass)" if fused else "slot-scan pipeline (k_decode, k_scan_blocks, k_pack_tma)"
         # roofline of the dominant kernel, from THIS rank's stage times
         dom = max(stages, key=stages.get)
@@ -781,7 +801,7 @@ def main():
         dom_alg = {"pack": pack_alg, "fused": pipe_alg}.get(dom, pipe_alg)
         achieved = dom_alg / (stages[dom] * 1e-3) / 1e9
         pipe_ms = sum(stages.values())                                                            # one pass alone (serial stages)
-        step_ms_rank0 = dev_ms / (steps * ppass)                                                  # with `depth` passes in flight
+        step_ms_rank0 = dev_ms / steps                                                            # with `depth` passes in flight
         mk_e2e = lambda ms_, m_: {"value": total_msgs / (ms_ * 1e-3), "unit": "msgs/s", "h2d_bytes_per_step": m_["h2d_bytes_per_step"],
                                   "d2h_bytes_per_step": m_["d2h_bytes_per_step"], "ms_per_step": ms_, "steps": m_["steps"]}
         e2e = mk_e2e(e_pull, e2e_modes["pull_by_ref"])
@@ -804,7 +824,7 @@ def main():
                                       "algorithmic_bytes_per_msg": pipe_alg / n_msgs, "single_pass_ms": pipe_ms, "launches_per_pass": int(launches_per_pass),
                                       "stage_ms": stages, "note": "whole hot path: (req + resp + 64 B desc) x msgs / measured time per pass"},
                 "latency": latency, "clocks": clocks, "wall_ms_per_step": wall_ms_max / steps,
-                "value_by_wall_clock": total_msgs * ppass * steps / (wall_ms_max * 1e-3), "msgs_per_step": total_msgs * ppass,
+                "value_by_wall_clock": total_msgs * steps / (wall_ms_max * 1e-3), "msgs_per_step": total_msgs,
                 "counters_allreduced": counters}
         if not use_dist and N_SOCKETS == 64 and args.run_mib >= 1:      # (the C++ bench has 64 connections of whole MiB)
             # the same e2e through the C++ host side a brpc transport would run (b2::GpuTransport: registered read regions, 8 groups of

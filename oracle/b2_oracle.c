@@ -10,7 +10,6 @@
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
-#include <dlfcn.h>
 
 /* ------------------------------------------------------------------------ */
 /* CRC-32C.  src/butil/crc32c.cc:379-454 (Extend: init/xorout 0xffffffff,
@@ -48,35 +47,145 @@ uint32_t orc_crc32c_mask(uint32_t crc) { return ((crc >> 15) | (crc << 17)) + 0x
 uint32_t orc_crc32c_unmask(uint32_t m) { uint32_t rot = m - 0xa282ead8u; return (rot >> 17) | (rot << 15); }
 
 /* ------------------------------------------------------------------------ */
-/* Snappy: the reference vendors Snappy 1.1.3 (src/butil/third_party/snappy).
- * The oracle calls the reference's own code compiled into oracle/_ref
- * (oracle/Makefile); raw-format helpers exported there:                     */
-typedef size_t (*ref_snappy_max_fn)(size_t);
-typedef int (*ref_snappy_compress_fn)(const char*, size_t, char*, size_t*);
-typedef int (*ref_snappy_uncompress_fn)(const char*, size_t, char*, size_t, size_t*);
-typedef int (*ref_snappy_ulen_fn)(const char*, size_t, size_t*);
-static void* g_ref = NULL;
-static ref_snappy_max_fn g_sn_max; static ref_snappy_compress_fn g_sn_c;
-static ref_snappy_uncompress_fn g_sn_u; static ref_snappy_ulen_fn g_sn_len;
-static int ref_load(void) {
-    if (g_ref) return 1;
-    const char* path = getenv("B2_ORACLE_REF");
-    Dl_info info; char buf[4096];
-    if (!path && dladdr((void*)&ref_load, &info) && info.dli_fname) {
-        snprintf(buf, sizeof buf, "%s", info.dli_fname);
-        char* slash = strrchr(buf, '/');
-        if (slash) { snprintf(slash + 1, sizeof buf - (size_t)(slash + 1 - buf), "_ref/libref_leaf.so"); path = buf; }
+/* Snappy raw format (format_description.txt of the snappy project), as the
+ * reference vendors it: Snappy 1.1.3 (src/butil/third_party/snappy).  The
+ * encoder follows that version's CompressFragment (snappy.cc:329-468): 64 KiB
+ * fragments, a zeroed uint16 hash table of 256..16384 entries (>= fragment
+ * size), hash = load32 * 0x1e35a7bd >> shift, skip heuristic skip++ >> 5, a
+ * 15-byte input margin, EmitLiteral / EmitCopy (:156-233); so its bytes are
+ * the reference's (pinned by tests/golden/snappy_vectors.json).  The decoder
+ * gives RawUncompress's verdict (snappy.cc:716-787, :1145-1215): well formed,
+ * input consumed exactly, exactly the announced length produced.             */
+size_t orc_snappy_max_compressed_length(size_t n) { return 32 + n + n / 6; }   /* snappy.cc:55-77 */
+
+static uint32_t sn_ld32(const uint8_t* p) { return (uint32_t)p[0] | ((uint32_t)p[1] << 8) | ((uint32_t)p[2] << 16) | ((uint32_t)p[3] << 24); }
+static size_t sn_literal(uint8_t* op, const uint8_t* src, size_t len) {
+    size_t n = len - 1, w = 1;
+    if (n < 60) op[0] = (uint8_t)(n << 2);
+    else {
+        uint32_t count = 0;
+        while (n > 0) { op[1 + count] = (uint8_t)(n & 0xff); n >>= 8; count++; }
+        op[0] = (uint8_t)((59 + count) << 2); w += count;
     }
-    if (!path) return 0;
-    g_ref = dlopen(path, RTLD_NOW | RTLD_LOCAL);
-    if (!g_ref) return 0;
-    g_sn_max = (ref_snappy_max_fn)dlsym(g_ref, "ref_snappy_max_compressed_length");
-    g_sn_c = (ref_snappy_compress_fn)dlsym(g_ref, "ref_snappy_compress");
-    g_sn_u = (ref_snappy_uncompress_fn)dlsym(g_ref, "ref_snappy_uncompress");
-    g_sn_len = (ref_snappy_ulen_fn)dlsym(g_ref, "ref_snappy_uncompressed_length");
-    return g_sn_max && g_sn_c && g_sn_u && g_sn_len;
+    memcpy(op + w, src, len);
+    return w + len;
 }
-int orc_have_ref(void) { return ref_load(); }
+static size_t sn_copy_lt64(uint8_t* op, size_t offset, size_t len) {
+    if (len < 12 && offset < 2048) { op[0] = (uint8_t)(1 + ((len - 4) << 2) + ((offset >> 8) << 5)); op[1] = (uint8_t)(offset & 0xff); return 2; }
+    op[0] = (uint8_t)(2 + ((len - 1) << 2)); op[1] = (uint8_t)(offset & 0xff); op[2] = (uint8_t)(offset >> 8); return 3;
+}
+static size_t sn_copy(uint8_t* op, size_t offset, size_t len) {
+    size_t w = 0;
+    while (len >= 68) { w += sn_copy_lt64(op + w, offset, 64); len -= 64; }
+    if (len > 64) { w += sn_copy_lt64(op + w, offset, 60); len -= 60; }
+    return w + sn_copy_lt64(op + w, offset, len);
+}
+static size_t sn_fragment(const uint8_t* in, size_t n, uint8_t* out, uint16_t* table) {
+    uint32_t table_size = 256, shift = 24;
+    while (table_size < 16384 && table_size < n) { table_size <<= 1; shift--; }
+    memset(table, 0, table_size * sizeof *table);
+    size_t op = 0, ip = 0, next_emit = 0;
+    if (n >= 15) {
+        const size_t ip_limit = n - 15;
+        uint32_t next_hash = (sn_ld32(in + 1) * 0x1e35a7bdu) >> shift;
+        ip = 1;
+        for (;;) {
+            size_t candidate, next_ip = ip;
+            uint32_t skip = 32;
+            for (;;) {                                               /* a 4-byte match */
+                ip = next_ip;
+                const uint32_t hash = next_hash;
+                next_ip = ip + (skip++ >> 5);
+                if (next_ip > ip_limit) goto emit_remainder;
+                next_hash = (sn_ld32(in + next_ip) * 0x1e35a7bdu) >> shift;
+                candidate = table[hash];
+                table[hash] = (uint16_t)ip;
+                if (sn_ld32(in + ip) == sn_ld32(in + candidate)) break;
+            }
+            op += sn_literal(out + op, in + next_emit, ip - next_emit);
+            for (;;) {                                               /* copies while the next position matches again */
+                const size_t base = ip;
+                size_t matched = 4;
+                while (ip + matched < n && in[candidate + matched] == in[ip + matched]) matched++;
+                ip += matched;
+                op += sn_copy(out + op, base - candidate, matched);
+                next_emit = ip;
+                if (ip >= ip_limit) goto emit_remainder;
+                table[(sn_ld32(in + ip - 1) * 0x1e35a7bdu) >> shift] = (uint16_t)(ip - 1);
+                const uint32_t cur = sn_ld32(in + ip), cur_hash = (cur * 0x1e35a7bdu) >> shift;
+                candidate = table[cur_hash];
+                table[cur_hash] = (uint16_t)ip;
+                if (cur != sn_ld32(in + candidate)) break;
+            }
+            next_hash = (sn_ld32(in + ip + 1) * 0x1e35a7bdu) >> shift;
+            ++ip;
+        }
+    }
+emit_remainder:
+    if (next_emit < n) op += sn_literal(out + op, in + next_emit, n - next_emit);
+    return op;
+}
+/* RawCompress: varint32 length, then the fragments; out holds orc_snappy_max_compressed_length(n) */
+size_t orc_snappy_compress(const uint8_t* in, size_t n, uint8_t* out) {
+    uint16_t table[16384];
+    size_t op = 0, v = n;
+    while (v >= 0x80) { out[op++] = (uint8_t)(v | 0x80); v >>= 7; }
+    out[op++] = (uint8_t)v;
+    for (size_t pos = 0; pos < n; pos += 65536) op += sn_fragment(in + pos, n - pos < 65536 ? n - pos : 65536, out + op, table);
+    return op;
+}
+/* GetUncompressedLength: the varint32 preamble (SnappyDecompressor::ReadUncompressedLength, snappy.cc:690-711) */
+static int sn_preamble(const uint8_t* in, size_t n, size_t* ulen, size_t* used) {
+    uint32_t v = 0, shift = 0; size_t ip = 0;
+    for (;;) {
+        if (shift >= 32 || ip >= n) return 0;
+        const uint32_t c = in[ip++];
+        v |= (c & 0x7f) << shift;
+        if (c < 128) break;
+        shift += 7;
+    }
+    *ulen = v; if (used) *used = ip;
+    return 1;
+}
+int orc_snappy_uncompressed_length(const uint8_t* in, size_t n, size_t* ulen) { return sn_preamble(in, n, ulen, NULL); }
+/* RawUncompress into out[cap]: 1 and *got = the announced length when the stream is valid and fits, else 0 */
+int orc_snappy_uncompress(const uint8_t* in, size_t n, uint8_t* out, size_t cap, size_t* got) {
+    size_t ulen, ip, op = 0;
+    if (!sn_preamble(in, n, &ulen, &ip) || ulen > cap) return 0;
+    while (ip < n) {
+        const uint32_t c = in[ip++];
+        if ((c & 3) == 0) {                                          /* literal */
+            uint64_t len = (c >> 2) + 1;
+            if (len >= 61) {
+                const size_t ll = len - 60;
+                if (n - ip < ll) return 0;
+                uint64_t v = 0;
+                for (size_t k = 0; k < ll; k++) v |= (uint64_t)in[ip + k] << (8 * k);
+                len = v + 1; ip += ll;
+            }
+            if (len > n - ip || len > ulen - op) return 0;           /* premature end of input / no room */
+            memcpy(out + op, in + ip, len); ip += len; op += len;
+        } else {                                                     /* copy */
+            size_t len, offset;
+            if ((c & 3) == 1) {
+                if (n - ip < 1) return 0;
+                len = ((c >> 2) & 7) + 4; offset = ((size_t)(c >> 5) << 8) | in[ip]; ip += 1;
+            } else if ((c & 3) == 2) {
+                if (n - ip < 2) return 0;
+                len = (c >> 2) + 1; offset = in[ip] | ((size_t)in[ip + 1] << 8); ip += 2;
+            } else {
+                if (n - ip < 4) return 0;
+                len = (c >> 2) + 1; offset = sn_ld32(in + ip); ip += 4;
+            }
+            if (offset == 0 || offset > op || len > ulen - op) return 0;
+            for (size_t i = 0; i < len; i++) out[op + i] = out[op - offset + i];     /* may overlap its own output */
+            op += len;
+        }
+    }
+    if (op != ulen) return 0;
+    *got = op;
+    return 1;
+}
 
 /* ------------------------------------------------------------------------ */
 /* protobuf wire reader: restates google::protobuf (pinned 27.3, MODULE.bazel:11)
@@ -345,15 +454,12 @@ static size_t serialize_echo_body(const uint8_t* msg, uint32_t len, int32_t comp
     size_t pb_len = 1 + varint_len(len) + len, body_len = 0;
     *cks_len = 0;
     if (compress_type == B2_COMPRESS_TYPE_SNAPPY) {
-        if (!ref_load()) return (size_t)-1;
         uint8_t* pb = (uint8_t*)malloc(pb_len ? pb_len : 1);
         wr_t w = { pb, pb + pb_len, 0 };
         wr_len(&w, 1, msg, len);
-        size_t olen = g_sn_max(pb_len);
-        if (olen > cap) { free(pb); return (size_t)-1; }
-        if (!g_sn_c((const char*)pb, pb_len, (char*)out, &olen)) { free(pb); return (size_t)-1; }
+        if (orc_snappy_max_compressed_length(pb_len) > cap) { free(pb); return (size_t)-1; }
+        body_len = orc_snappy_compress(pb, pb_len, out);
         free(pb);
-        body_len = olen;
     } else {
         wr_t w = { out, out + cap, 0 };
         wr_len(&w, 1, msg, len);
@@ -595,11 +701,8 @@ size_t orc_pack_response(const b2_reply* r, const uint8_t* bytes, uint8_t* out, 
     const uint8_t* cks = bytes + r->checksum_value_off; size_t cks_len = r->checksum_value_len;
     if (append_body) {
         if (r->compress_type == B2_COMPRESS_TYPE_SNAPPY) {
-            if (!ref_load()) return 0;
-            size_t olen = g_sn_max(r->body_len);
-            body = (uint8_t*)malloc(olen ? olen : 1);
-            if (!g_sn_c((const char*)bytes + r->body_off, r->body_len, (char*)body, &olen)) { free(body); return 0; }
-            body_len = olen;
+            body = (uint8_t*)malloc(orc_snappy_max_compressed_length(r->body_len));
+            body_len = orc_snappy_compress(bytes + r->body_off, r->body_len, body);
         } else { body = (uint8_t*)malloc(r->body_len ? r->body_len : 1); memcpy(body, bytes + r->body_off, r->body_len); body_len = r->body_len; }
         if (r->checksum_type == B2_CHECKSUM_TYPE_CRC32C) {
             const uint32_t c = orc_crc32c_mask(orc_crc32c_extend(0, body, body_len));
@@ -763,12 +866,11 @@ static int process_rpc_request(const orc_config* cfg, const uint8_t* frame, b2_m
             if (m.compress_type == B2_COMPRESS_TYPE_NONE) {
             } else if (m.compress_type == B2_COMPRESS_TYPE_SNAPPY) {         /* SnappyDecompress, snappy_compress.cpp:51-70 */
                 size_t ulen = 0;
-                if (!ref_load()) { d->status = B2_MSG_UNSUPPORTED; return 0; }
-                if (!g_sn_len((const char*)req_buf, req_buf_len, &ulen)) ok = 0;
+                if (!orc_snappy_uncompressed_length(req_buf, req_buf_len, &ulen)) ok = 0;
                 else {
                     unz = (uint8_t*)malloc(ulen ? ulen : 1);
                     size_t got = 0;
-                    if (!g_sn_u((const char*)req_buf, req_buf_len, (char*)unz, ulen, &got)) ok = 0;
+                    if (!orc_snappy_uncompress(req_buf, req_buf_len, unz, ulen, &got)) ok = 0;
                     pb = unz; pb_len = got;
                 }
             } else if (m.compress_type == B2_COMPRESS_TYPE_GZIP || m.compress_type == B2_COMPRESS_TYPE_ZLIB) {
@@ -859,9 +961,8 @@ static int process_rpc_response(const uint8_t* frame, b2_msg_desc* d, uint8_t* r
         if (ok) { d->resp_off = d->frame_off + 12 + d->meta_size + msg.off; d->resp_len = msg.len; }
     } else if (ok && m.compress_type == B2_COMPRESS_TYPE_SNAPPY) {
         size_t ulen = 0, got = 0;
-        if (!ref_load()) { d->status = B2_MSG_UNSUPPORTED; return 0; }
-        if (!g_sn_len((const char*)payload, body_len, &ulen) || ulen > 32 * (uint64_t)body_len + 64 || ulen > resp_cap) ok = 0;
-        else if (!g_sn_u((const char*)payload, body_len, (char*)resp, ulen, &got)) ok = 0;
+        if (!orc_snappy_uncompressed_length(payload, body_len, &ulen) || ulen > 32 * (uint64_t)body_len + 64 || ulen > resp_cap) ok = 0;
+        else if (!orc_snappy_uncompress(payload, body_len, resp, ulen, &got)) ok = 0;
         else ok = orc_parse_echo_request(resp, got, &msg);
         if (ok) { d->status = B2_MSG_RESPONSE_UNZ; *resp_len = got; d->resp_len = msg.len; d->resp_off = msg.off; /* + slot, by caller */ }
     } else if (ok && (m.compress_type == B2_COMPRESS_TYPE_GZIP || m.compress_type == B2_COMPRESS_TYPE_ZLIB)) {
@@ -890,8 +991,8 @@ static void process_stream_frame(const orc_config* cfg, const uint8_t* frame, b2
         /* policy::SnappyDecompress(IOBuf, IOBuf), snappy_compress.cpp:77-82, on the frame payload */
         const uint8_t* data = frame + 12 + d->meta_size; const size_t n = d->body_size - d->meta_size;
         size_t ulen = 0, got = 0;
-        if (!ref_load() || !g_sn_len((const char*)data, n, &ulen) || ulen > 32 * (uint64_t)n + 64 || ulen > resp_cap ||
-            !g_sn_u((const char*)data, n, (char*)resp, ulen, &got)) { d->error_code = B2_EREQUEST; return; }
+        if (!orc_snappy_uncompressed_length(data, n, &ulen) || ulen > 32 * (uint64_t)n + 64 || ulen > resp_cap ||
+            !orc_snappy_uncompress(data, n, resp, ulen, &got)) { d->error_code = B2_EREQUEST; return; }
         *resp_len = got;
     }
 }

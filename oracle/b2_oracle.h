@@ -12,7 +12,9 @@
  * compiled into oracle/_ref; the protobuf wire codec (libprotobuf is a
  * third-party dependency absent from /root/reference, pinned 27.3 in
  * MODULE.bazel:11) is pinned by tests/golden/ (json) generated with
- * python-protobuf from the reference's .proto files (tests/golden/gen_golden.py).
+ * python-protobuf from the reference's .proto files (tests/golden/gen_golden.py);
+ * snappy by the vendored snappy's compressed bytes and decoder verdicts
+ * (tests/golden/snappy_vectors.json, snappy_ref_results.json).
  * The reference's tests hold NO golden baidu_std wire bytes (SURVEY §8c), so
  * frame-level parity is pinned by those fixtures, not by reference test vectors.
  */
@@ -76,6 +78,10 @@ typedef struct orc_config {
 uint32_t orc_crc32c_extend(uint32_t init_crc, const void* data, size_t n); /* crc32c.cc:379-454 */
 uint32_t orc_crc32c_mask(uint32_t crc);                                      /* crc32c.h:38-41 */
 uint32_t orc_crc32c_unmask(uint32_t masked);                                 /* crc32c.h:44-47 */
+size_t orc_snappy_max_compressed_length(size_t n);                            /* snappy.cc:55-77 */
+size_t orc_snappy_compress(const uint8_t* in, size_t n, uint8_t* out);        /* RawCompress, snappy.cc:875-956 */
+int orc_snappy_uncompressed_length(const uint8_t* in, size_t n, size_t* ulen); /* GetUncompressedLength */
+int orc_snappy_uncompress(const uint8_t* in, size_t n, uint8_t* out, size_t cap, size_t* got);  /* RawUncompress, cap >= length */
 
 /* ---- protobuf wire decode of the path's messages --------------------------
  * return 1 = ParsePbFromIOBuf succeeded (protocol.cpp:236-239), 0 = failed. */

@@ -80,7 +80,10 @@ lib.orc_pack_stream_frame.restype = C.c_size_t
 lib.orc_pack_stream_frame.argtypes = [C.c_int64, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_char_p, C.c_uint32, C.c_void_p, C.c_size_t]
 lib.orc_process_batch.argtypes = [C.POINTER(Config), C.c_void_p, C.c_uint32, C.c_void_p, C.c_uint32, C.c_void_p,
                                   C.c_void_p, C.c_uint32, C.POINTER(C.c_uint32), C.c_void_p, C.c_uint32, C.POINTER(C.c_uint32)]
-lib.orc_have_ref.restype = C.c_int
+lib.orc_snappy_max_compressed_length.restype = C.c_size_t; lib.orc_snappy_max_compressed_length.argtypes = [C.c_size_t]
+lib.orc_snappy_compress.restype = C.c_size_t; lib.orc_snappy_compress.argtypes = [C.c_char_p, C.c_size_t, C.c_void_p]
+lib.orc_snappy_uncompressed_length.argtypes = [C.c_char_p, C.c_size_t, C.POINTER(C.c_size_t)]
+lib.orc_snappy_uncompress.argtypes = [C.c_char_p, C.c_size_t, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)]
 
 
 lib.orc_gzip_input_stream.argtypes = [C.c_char_p, C.c_size_t, C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t)]
@@ -109,6 +112,25 @@ def gzip_input_stream(b, fmt):
     r = C.string_at(out, n.value)
     lib.orc_free(out)
     return r
+
+
+def snappy_compress(b):
+    """RawCompress of the reference's snappy 1.1.3 (the oracle's restatement, pinned by tests/golden/snappy_vectors.json)."""
+    out = C.create_string_buffer(lib.orc_snappy_max_compressed_length(len(b)))
+    n = lib.orc_snappy_compress(bytes(b), len(b), out)
+    return out.raw[:n]
+
+
+def snappy_uncompressed_length(b):
+    """GetUncompressedLength: the announced length, or None when the preamble is malformed."""
+    n = C.c_size_t()
+    return n.value if lib.orc_snappy_uncompressed_length(bytes(b), len(b), C.byref(n)) else None
+
+
+def snappy_uncompress(b, cap):
+    """RawUncompress: the bytes, or None when the stream is invalid or announces more than cap bytes."""
+    out = C.create_string_buffer(max(1, cap)); got = C.c_size_t()
+    return out.raw[:got.value] if lib.orc_snappy_uncompress(bytes(b), len(b), out, cap, C.byref(got)) else None
 
 
 def crc32c(b, init=0):

@@ -1,8 +1,8 @@
 """CPU: the WARP-cooperative device code of the hot path — warp_crc32c_update, warp_snappy_decode / _compress, pack_one — on an emulated 32-lane
 warp (tests/cpp/warp_emul_prelude.h: 32 host threads, every __shfl / __ballot / __syncwarp a barrier plus an exchange), out of the generated
-host-compilable copy of b2_kernels.cuh.  CRC against the oracle (which the reference's crc32c.cc pins), snappy against the reference's vendored
-snappy (oracle/_ref), and whole batches — decode_one per message, slot scan, pack_one per message — against the oracle's descriptors and reply
-bytes for every kind of message (errors, CRC32C, snappy and gzip / zlib requests, snappy replies, attachments, client sockets, stream frames)."""
+host-compilable copy of b2_kernels.cuh.  CRC against the oracle (which the reference's crc32c.cc pins), snappy against what the reference's
+vendored snappy returned for the same inputs (tests/golden/snappy_ref_results.json), and whole batches — decode_one per message, slot scan,
+pack_one per message — against the oracle's descriptors and reply bytes for every kind of message (errors, CRC32C, snappy and gzip / zlib requests, snappy replies, attachments, client sockets, stream frames)."""
 import ctypes as C
 import os
 import random
@@ -23,6 +23,7 @@ from _traffic import SEED, echo_frame, echo_pb, mixed_frames, raw_request_frame,
 from brpc_b200.abi import ECHO_METHOD, MSG_DT  # noqa: E402
 from brpc_b200.messenger import make_runs  # noqa: E402
 from _compare import MSG_FIELDS  # noqa: E402
+import _snappy_cases as S  # noqa: E402
 
 
 @pytest.fixture(scope="module")
@@ -64,42 +65,27 @@ def test_warp_crc32c_against_the_oracle(wh):
 
 
 def test_warp_snappy_against_the_reference_library(wh):
-    ref = C.CDLL(os.path.join(ROOT, "oracle", "_ref", "libref_leaf.so"))
-    ref.ref_snappy_max_compressed_length.restype = C.c_size_t
-    ref.ref_snappy_max_compressed_length.argtypes = [C.c_size_t]
-    ref.ref_snappy_compress.argtypes = [C.c_char_p, C.c_size_t, C.c_char_p, C.POINTER(C.c_size_t)]
-    ref.ref_snappy_uncompress.argtypes = [C.c_char_p, C.c_size_t, C.c_char_p, C.c_size_t, C.POINTER(C.c_size_t)]
-    ref.ref_snappy_uncompressed_length.argtypes = [C.c_char_p, C.c_size_t, C.POINTER(C.c_size_t)]
+    want = S.ref_results()["warp"]["long" if LONG else "short"]
+    corrupt = iter(want["corrupt"])
     rng = random.Random(SEED + 972)
-    text = b" ".join(rng.choice([b"echo", b"brpc", b"socket", b"iobuf", b"x" * 30]) for _ in range(4000))
-    raws = [b"", b"a", b"abcd" * 10, rnd62(rng, 100), rnd62(rng, 5000), text, text * 5, b"\x00" * 70000, rnd62(rng, 70000), (rnd62(rng, 37) * 3000)[:100000]] if LONG else \
-           [b"", b"a", b"abcd" * 10, rnd62(rng, 100), rnd62(rng, 3000), text[:20000], b"\x00" * 9000, (rnd62(rng, 37) * 300)[:9000], rnd62(rng, 70000)[:20000]]
-    for raw in raws:
-        cap = ref.ref_snappy_max_compressed_length(len(raw)); want = C.create_string_buffer(cap); wl = C.c_size_t(cap)
-        ref.ref_snappy_compress(raw, len(raw), want, C.byref(wl))
-        out = C.create_string_buffer(cap + 64)
+    for raw, want_comp in zip(S.warp_raws(rng, LONG), want["compress"]):
+        out = C.create_string_buffer(len(raw) + len(raw) // 6 + 96)
         n = wh.wh_snappy_compress(raw, len(raw), out)
-        assert n == wl.value and out.raw[:n] == want.raw[:n], len(raw)                          # bit-exact with the vendored snappy 1.1.3
+        assert S.digest(out.raw[:n]) == want_comp, len(raw)                                      # bit-exact with the vendored snappy 1.1.3
         back = C.create_string_buffer(max(1, len(raw))); prod = C.c_uint32()
         assert wh.wh_snappy_uncompress(out.raw[:n], n, back, len(raw), C.byref(prod)) == 1 and back.raw[:prod.value] == raw
-        for _ in range(30 if LONG else 12):                                                       # corrupted streams: the reference's verdict
-            b = bytearray(out.raw[:n])
-            if not b: break
-            c = rng.random()
-            if c < 0.3: del b[rng.randrange(len(b)):]
-            elif c < 0.8: b[rng.randrange(len(b))] ^= 1 << rng.randrange(8)
-            else: b += bytes(rng.getrandbits(8) for _ in range(3))
-            ul = C.c_size_t()
-            ok_len = ref.ref_snappy_uncompressed_length(bytes(b), len(b), C.byref(ul))
-            if not ok_len or ul.value > 32 * len(b) + 64 or ul.value > (1 << 20):
+        for _ in range(S.warp_corruptions_per_raw(LONG)):                                       # corrupted streams: the reference's verdict
+            if not n: break
+            b = S.warp_corruption(rng, out.raw[:n])
+            ul, ok_ref, want_out = next(corrupt)
+            if ok_ref is None:
                 continue
-            wbuf = C.create_string_buffer(max(1, ul.value)); got = C.c_size_t()
-            ok_ref = ref.ref_snappy_uncompress(bytes(b), len(b), wbuf, ul.value, C.byref(got))
-            dbuf = C.create_string_buffer(max(1, ul.value)); prod = C.c_uint32()
-            ok_dev = wh.wh_snappy_uncompress(bytes(b), len(b), dbuf, ul.value, C.byref(prod))
+            dbuf = C.create_string_buffer(max(1, ul)); prod = C.c_uint32()
+            ok_dev = wh.wh_snappy_uncompress(b, len(b), dbuf, ul, C.byref(prod))
             assert ok_dev == (1 if ok_ref else 0), (len(raw), len(b))
             if ok_ref:
-                assert dbuf.raw[:prod.value] == wbuf.raw[:got.value]
+                assert S.digest(dbuf.raw[:prod.value]) == want_out
+    assert next(corrupt, None) is None
 
 
 def _process(wh, k, cfg, chunks, flags=0):
@@ -136,7 +122,6 @@ def _make(wh, methods, identity=None, stream_handler=0):
 
 
 def test_decode_and_pack_of_whole_batches_on_the_emulated_warp(wh):
-    assert O.lib.orc_have_ref()
     rng = random.Random(SEED + 973)
     total = 0
     for r_cks, r_cmp, identity in [(0, 0, None), (1, 0, b"10.0.0.1:8000"), (0, 1, None), (1, 1, None)]:
@@ -181,11 +166,7 @@ def test_client_sockets_and_stream_payloads_on_the_emulated_warp(wh):
     n_frames = 40 if LONG else 18
     for i in range(n_frames):
         raw = rng.choice([rnd62(rng, rng.choice([0, 100, 30000] if LONG else [0, 100, 4000])), b"z" * (5000 if LONG else 1500)])
-        cap = 32 + len(raw) + len(raw) // 6 + 64
-        ref = C.CDLL(os.path.join(ROOT, "oracle", "_ref", "libref_leaf.so"))
-        ref.ref_snappy_compress.argtypes = [C.c_char_p, C.c_size_t, C.c_char_p, C.POINTER(C.c_size_t)]
-        outb = C.create_string_buffer(cap); ol = C.c_size_t(cap); ref.ref_snappy_compress(raw, len(raw), outb, C.byref(ol))
-        payload = outb.raw[:ol.value]
+        payload = O.snappy_compress(raw)
         if rng.random() < 0.2 and payload:
             b = bytearray(payload); b[rng.randrange(len(b))] ^= 4; payload = bytes(b)
         frames.append(O.pack_stream_frame(1000 + i, -1, 3, None, payload))

@@ -1,41 +1,36 @@
-"""GPU: the reference-signature leaves of seam 4 (b2_crc32c_extend, b2_snappy_raw_compress / _raw_uncompress, ...) against the
-reference's own crc32c.cc and vendored snappy compiled unmodified into oracle/_ref/libref_leaf.so."""
+"""GPU: the reference-signature leaves of seam 4 (b2_crc32c_extend, b2_snappy_raw_compress / _raw_uncompress, ...) against what the
+reference's own crc32c.cc and vendored snappy return for the same inputs (tests/golden/snappy_ref_results.json)."""
 import ctypes as C
-import os
 import random
 
 import pytest
 
+import _snappy_cases as S
+
 pytestmark = pytest.mark.gpu
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def test_reference_signature_leaves_match_the_reference_build():
     import brpc_b200
     lib = brpc_b200.lib
-    ref = C.CDLL(os.path.join(ROOT, "oracle", "_ref", "libref_leaf.so"))
-    ref.ref_crc32c_extend.restype = C.c_uint32; ref.ref_crc32c_extend.argtypes = [C.c_uint32, C.c_char_p, C.c_size_t]
-    ref.ref_snappy_max_compressed_length.restype = C.c_size_t; ref.ref_snappy_max_compressed_length.argtypes = [C.c_size_t]
-    ref.ref_snappy_compress.argtypes = [C.c_char_p, C.c_size_t, C.c_char_p, C.POINTER(C.c_size_t)]
     rng = random.Random(20260921)
-    t62 = b"abcdefghijklmnopqrstuvwxyzABCDEFGHIJKLMNOPQRSTUVWXYZ0123456789"
-    for n in [0, 1, 7, 47, 48, 100, 1027, 4099, 70001, 300000]:
-        raw = bytes(rng.choice(t62) for _ in range(min(n, 5000))) * (n // 5000 + 1)
-        raw = raw[:n]
+    want = S.ref_results()["leaf"]
+    assert [w["n"] for w in want] == S.LEAF_SIZES
+    for w in want:
+        n = w["n"]
+        raw = S.leaf_raw(rng, n)
         # Extend chains: crc(a + b) == Extend(Extend(0, a), b)
         cut = n // 3
-        want = ref.ref_crc32c_extend(ref.ref_crc32c_extend(0, raw[:cut], cut), raw[cut:], n - cut)
         got = lib.b2_crc32c_extend(lib.b2_crc32c_extend(0, raw[:cut], cut), raw[cut:], n - cut)
-        assert got == want == ref.ref_crc32c_extend(0, raw, n), n
-        assert lib.b2_snappy_max_compressed_length(n) == ref.ref_snappy_max_compressed_length(n)
-        cap = ref.ref_snappy_max_compressed_length(n)
-        a = C.create_string_buffer(cap + 16); an = C.c_size_t(cap)
-        ref.ref_snappy_compress(raw, n, a, C.byref(an))
+        assert got == w["crc32c"] == lib.b2_crc32c_extend(0, raw, n), n
+        cap = lib.b2_snappy_max_compressed_length(n)
+        assert cap == w["max_compressed_length"]
         b = C.create_string_buffer(cap + 16); bn = C.c_size_t(0)
         lib.b2_snappy_raw_compress(raw, n, b, C.byref(bn))
-        assert bn.value == an.value and b.raw[:bn.value] == a.raw[:an.value], "snappy bytes differ at n=%d" % n
+        comp = b.raw[:bn.value]
+        assert S.digest(comp) == w["compressed"], "snappy bytes differ at n=%d" % n
         ul = C.c_size_t(0)
-        assert lib.b2_snappy_get_uncompressed_length(a.raw[:an.value], an.value, C.byref(ul)) == 1 and ul.value == n
+        assert lib.b2_snappy_get_uncompressed_length(comp, len(comp), C.byref(ul)) == 1 and ul.value == n
         out = C.create_string_buffer(n + 16)
-        assert lib.b2_snappy_raw_uncompress(a.raw[:an.value], an.value, out) == 1 and out.raw[:n] == raw
+        assert lib.b2_snappy_raw_uncompress(comp, len(comp), out) == 1 and out.raw[:n] == raw
     assert lib.b2_snappy_raw_uncompress(b"\x05abc", 4, C.create_string_buffer(64)) == 0       # malformed stream: false, like the reference

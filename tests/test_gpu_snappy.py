@@ -1,10 +1,9 @@
 """GPU: snappy decode (a10).  (1) the leaf b2_snappy_uncompress_batch against the golden vectors
 produced by the reference's vendored snappy (tests/golden/snappy_vectors.json, patterns of
-test/brpc_snappy_compress_unittest.cpp:80-255) and against the reference decoder itself on
-corrupted streams; (2) snappy-compressed baidu_std requests through the whole path vs the oracle
-(the compress x checksum matrix of test/brpc_server_unittest.cpp:1690-1880 restricted to
+test/brpc_snappy_compress_unittest.cpp:80-255) and against the reference decoder's results on
+corrupted streams (tests/golden/snappy_ref_results.json); (2) snappy-compressed baidu_std requests
+through the whole path vs the oracle (the compress x checksum matrix of test/brpc_server_unittest.cpp:1690-1880 restricted to
 {none, snappy} x {none, crc32c})."""
-import ctypes as C
 import json
 import os
 import random
@@ -14,35 +13,16 @@ import pytest
 
 pytestmark = pytest.mark.gpu
 HERE = os.path.dirname(os.path.abspath(__file__))
-ROOT = os.path.dirname(HERE)
 
 import _oracle as O  # noqa: E402
 from _compare import assert_same  # noqa: E402
 from _traffic import SEED, echo_frame, rnd62  # noqa: E402
+import _snappy_cases as S  # noqa: E402
 
 
 def _pattern(n):
     t = b"abcdefghijklmnopqrstuvwxyz0123456789"
     return (t * (n // len(t) + 1))[:n]
-
-
-def _ref():
-    ref = C.CDLL(os.path.join(ROOT, "oracle", "_ref", "libref_leaf.so"))
-    ref.ref_snappy_uncompress.argtypes = [C.c_char_p, C.c_size_t, C.c_char_p, C.c_size_t, C.POINTER(C.c_size_t)]
-    ref.ref_snappy_uncompressed_length.argtypes = [C.c_char_p, C.c_size_t, C.POINTER(C.c_size_t)]
-    return ref
-
-
-def ref_uncompress(ref, b):
-    ul = C.c_size_t(0)
-    if not ref.ref_snappy_uncompressed_length(b, len(b), C.byref(ul)):
-        return None
-    if ul.value > 32 * len(b) + 64:
-        return None            # cannot decode to that length (and would only allocate); reference returns false too
-    out = C.create_string_buffer(max(1, ul.value)); got = C.c_size_t(0)
-    if not ref.ref_snappy_uncompress(b, len(b), out, ul.value, C.byref(got)):
-        return None
-    return out.raw[:got.value]
 
 
 def test_snappy_golden_vectors_and_corruptions():
@@ -55,30 +35,23 @@ def test_snappy_golden_vectors_and_corruptions():
         raw = bytes.fromhex(v["raw_hex"]) if "raw_hex" in v else _pattern(v["raw_len"])
         assert len(raw) == v["raw_len"]
         blobs.append(comp); want.append(raw)
-    # corruptions: truncations, bit flips, bad offsets; expectation = the reference decoder's verdict
-    ref = _ref()
+    # corruptions: truncations, bit flips, bad offsets; expectation = the reference decoder's verdict (digest of its output)
     rng = random.Random(SEED)
     seeds = [b for b in blobs if 0 < len(b) < 5000]
-    for _ in range(400):
-        b = bytearray(rng.choice(seeds)); c = rng.random()
-        if c < 0.3: del b[rng.randrange(len(b)):]
-        elif c < 0.7:
-            for _k in range(rng.randrange(1, 4)): b[rng.randrange(len(b))] ^= 1 << rng.randrange(8)
-        elif c < 0.85: b += bytes(rng.randrange(256) for _k in range(rng.randrange(1, 5)))
-        else: b[rng.randrange(len(b))] = rng.randrange(256)
-        blobs.append(bytes(b)); want.append(ref_uncompress(ref, bytes(b)))
+    blobs += S.corrupted_blobs(rng, seeds)
     buf = bytearray(); offs = []; lens = []
     for b in blobs:
         buf += b"\x00" * rng.randrange(0, 5); offs.append(len(buf)); lens.append(len(b)); buf += b
     got = ctx.snappy_uncompress_batch(np.frombuffer(bytes(buf), np.uint8), offs, lens, 48 << 20)
-    bad = [i for i in range(len(blobs)) if got[i] != want[i]]
+    want = [S.digest(w) for w in want] + S.ref_results()["gpu_corruptions"]
+    assert len(want) == len(blobs)
+    bad = [i for i in range(len(blobs)) if S.digest(got[i]) != want[i]]
     assert not bad, "mismatch at %s (want None? %s)" % (bad[:5], [want[i] is None for i in bad[:5]])
     assert sum(w is None for w in want) > 50 and sum(w is not None for w in want[len(vec):]) > 5
 
 
 def test_snappy_requests_through_the_path():
     import brpc_b200
-    assert O.lib.orc_have_ref(), "oracle/_ref missing (reference snappy)"
     rng = random.Random(SEED + 1)
     ms = [dict(brpc_b200.ECHO_METHOD, response_checksum_type=rng.choice([0, 1]))]
     for tile in (512, 8192):
@@ -152,19 +125,10 @@ def test_snappy_replies_through_the_path():
         assert (dev[1]["status"] == 0).sum() > 50
 
 
-def _ref_compress(ref, raw):
-    ref.ref_snappy_max_compressed_length.restype = C.c_size_t; ref.ref_snappy_max_compressed_length.argtypes = [C.c_size_t]
-    ref.ref_snappy_compress.argtypes = [C.c_char_p, C.c_size_t, C.c_char_p, C.POINTER(C.c_size_t)]
-    cap = ref.ref_snappy_max_compressed_length(len(raw)); out = C.create_string_buffer(cap); n = C.c_size_t(cap)
-    ref.ref_snappy_compress(raw, len(raw), out, C.byref(n))
-    return out.raw[:n.value]
-
-
 def test_streaming_frames_with_snappy_payloads():
     """BASELINE configs[4] shape: streaming_rpc DATA frames whose payloads the application snappy-compressed
     (policy::SnappyCompress), cut + meta-decoded + decompressed on the device, interleaved with baidu_std calls."""
     import brpc_b200
-    ref = _ref()
     rng = random.Random(SEED + 3)
     ctx = brpc_b200.Context(device=0, max_batch_bytes=64 << 20, max_msgs=1 << 16, max_runs=256, stream_handler=1)
     cfg = O.make_config(stream_handler=1)
@@ -174,7 +138,7 @@ def test_streaming_frames_with_snappy_payloads():
         for i in range(rng.randrange(1, 8)):
             n = rng.choice([0, 10, 1000, 70000, 262144])
             raw = rng.choice([_pattern(n), rnd62(rng, min(n, 30000)), (rnd62(rng, 64) * (n // 64 + 1))[:n]])
-            comp = _ref_compress(ref, raw)
+            comp = O.snappy_compress(raw)
             if rng.random() < 0.15 and len(comp) > 4:
                 comp = bytearray(comp); comp[rng.randrange(len(comp))] ^= 0x10; comp = bytes(comp)
             fr.append(O.pack_stream_frame(1000 + s, 2000 + s, rng.choice([3, 3, 3, 4, 1]), rng.choice([None, False]), comp))

@@ -36,6 +36,29 @@ def test_crc32c_kat(oracle):
             assert oracle.lib.orc_crc32c_unmask(k["masked"]) == k["crc"]
 
 
+def test_snappy_matches_the_reference_results(oracle):
+    """The oracle's snappy against the vendored snappy 1.1.3: compressed bytes of snappy_vectors.json, RawUncompress's
+    verdict and output on the corrupted streams of snappy_ref_results.json."""
+    import random
+    import _snappy_cases as S
+    from _traffic import SEED
+    seeds = []
+    for v in load("snappy_vectors.json"):
+        raw = bytes.fromhex(v["raw_hex"]) if "raw_hex" in v else (b"abcdefghijklmnopqrstuvwxyz0123456789" * (v["raw_len"] // 36 + 1))[:v["raw_len"]]
+        comp = bytes.fromhex(v["comp_hex"])
+        assert oracle.snappy_compress(raw) == comp, v["name"]
+        assert oracle.snappy_uncompressed_length(comp) == len(raw) and oracle.snappy_uncompress(comp, len(raw)) == raw, v["name"]
+        if 0 < len(comp) < 5000:
+            seeds.append(comp)
+    want = S.ref_results()["gpu_corruptions"]
+    blobs = S.corrupted_blobs(random.Random(SEED), seeds)
+    assert len(blobs) == len(want)
+    for b, w in zip(blobs, want):
+        ul = oracle.snappy_uncompressed_length(b)
+        got = oracle.snappy_uncompress(b, ul) if ul is not None and ul <= 32 * len(b) + 64 else None
+        assert S.digest(got) == w, b.hex()[:80]
+
+
 def span(b, s):
     return b[s.off:s.off + s.len].hex()
 

