@@ -33,6 +33,8 @@ H2_REQUEST_DT = np.dtype([("conn", "<u4"), ("flags", "<u4"), ("path_off", "<u4")
                           ("body_len", "<u4"), ("extra_off", "<u4"), ("extra_len", "<u4")])          # == b2_h2_request, 48 bytes
 H2_PEER_UPDATE_DT = np.dtype([("set", "<u4"), ("header_table_size", "<u4"), ("max_frame_size", "<u4"), ("stream_window_size", "<u4"), ("conn_window_add", "<i8")])
 H2_REQUEST_RESULT_DT = np.dtype([("status", "<i4"), ("stream_id", "<u4"), ("out_off", "<u4"), ("out_len", "<u4")])
+H2_UNZ_RESULT_DT = np.dtype([("status", "<u4"), ("out_off", "<u4"), ("out_len", "<u4"), ("reserved", "<u4")])        # == b2_h2_unz_result
+H2_UNZ_NONE, H2_UNZ_OK, H2_UNZ_NO_ENCODING, H2_UNZ_NOT_GZIP, H2_UNZ_FAILED, H2_UNZ_HOST, H2_UNZ_NO_ROOM = range(7)
 H2_MSG_DT = np.dtype([("run_idx", "<u4"), ("stream_id", "<u4"), ("headers_off", "<u4"), ("headers_len", "<u4"), ("n_headers", "<u4"),
                       ("body_off", "<u4"), ("body_len", "<u4"), ("http_method", "<u4"), ("content_type", "<u4"), ("flags", "<u4"),
                       ("method_idx", "<i4"), ("msg_off", "<u4"), ("msg_len", "<u4"), ("path_off", "<u4"), ("path_len", "<u4"), ("reserved", "<u4")])
@@ -133,6 +135,7 @@ def _load():
     l.b2_h2_conn_set_next_stream_id.argtypes = [C.c_void_p, C.c_uint32, C.c_uint32]
     l.b2_h2_conn_peer_update.argtypes = [C.c_void_p, C.c_uint32, C.c_void_p]
     l.b2_h2_pack_responses.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_uint32, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p]
+    l.b2_h2_decompress_requests.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_uint32, C.c_void_p]
     l.b2_pack_requests.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_uint32, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p]
     l.b2_pack_responses.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_uint32, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p]
     l.b2_counters_read.argtypes = [C.c_void_p, C.POINTER(C.c_int64)]
@@ -147,7 +150,8 @@ ABI_SYMBOLS = ["b2_ctx_create", "b2_ctx_destroy", "b2_last_error", "b2_version",
                "b2_set_server_identity", "b2_set_stream_handler", "b2_set_protocols", "b2_block_alloc", "b2_block_free", "b2_block_pool_host_allocs", "b2_set_modes", "b2_ring_start", "b2_ring_stop", "b2_ring_submit", "b2_ring_wait", "b2_ring_launches", "b2_ring_phase_ns", "b2_latency_probe", "b2_process_batch", "b2_batch_submit", "b2_batch_collect", "b2_batch_upload",
                "b2_batch_execute", "b2_batch_execute_many", "b2_batch_download", "b2_batch_launch", "b2_batch_wait",
                "b2_elapsed_ms", "b2_batch_info", "b2_device_pci_bus_id", "b2_stage_times", "b2_crc32c_batch", "b2_crc32c_extend", "b2_snappy_max_compressed_length", "b2_snappy_raw_compress", "b2_snappy_get_uncompressed_length", "b2_snappy_raw_uncompress", "b2_snappy_uncompress_batch", "b2_snappy_compress_batch", "b2_hpack_reset", "b2_hpack_decode_batch", "b2_pack_requests", "b2_pack_responses", "b2_h2_scan_batch", "b2_h2_conn_reset", "b2_h2_configure", "b2_h2_process_batch", "b2_h2_pack_responses", "b2_counters_read",
-               "b2_counters_device_ptr", "b2_counters_allreduce", "b2_h2_pack_requests", "b2_h2_conn_set_next_stream_id", "b2_h2_conn_peer_update"]
+               "b2_counters_device_ptr", "b2_counters_allreduce", "b2_h2_pack_requests", "b2_h2_conn_set_next_stream_id", "b2_h2_conn_peer_update",
+               "b2_h2_decompress_requests"]
 
 ECHO_METHOD = dict(service_full_name=b"example.EchoService", service_name=b"EchoService", method_name=b"Echo",
                    request_type_name=b"example.EchoRequest", handler=1, echo_attachment=1,
@@ -447,6 +451,17 @@ class Context:
         if raw:
             return out, offs, lens
         return [out[offs[i]:offs[i] + lens[i]].tobytes() for i in range(n)]
+
+    def h2_decompress_requests(self, msgs, out_cap=None, out=None):
+        """GzipDecompress of ProcessHttpRequest for messages of the last h2_process_batch (its H2_MSG_DT records, in the order to
+        serve them).  Returns (H2_UNZ_RESULT_DT per message, out): an inflated message is out[out_off:out_off + out_len]."""
+        msgs = np.ascontiguousarray(msgs, dtype=H2_MSG_DT)
+        n = len(msgs)
+        if out is None:
+            out = np.empty(out_cap or (4 << 20), np.uint8)
+        res = np.zeros(n, H2_UNZ_RESULT_DT)
+        _check(lib.b2_h2_decompress_requests(self._h, msgs.ctypes.data, n, out.ctypes.data, out.nbytes, res.ctypes.data))
+        return res, out
 
     def h2_pack_requests(self, data, reqs, out_cap=None):
         """Client side of h2 (H2UnsentRequest): reqs is an H2_REQUEST_DT array (offsets into data).  Returns (results, [bytes per request])."""

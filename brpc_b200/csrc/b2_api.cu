@@ -7,6 +7,7 @@
 #include <time.h>
 #include <stdlib.h>
 #include <string.h>
+#include <algorithm>
 #include <mutex>
 #include <string>
 #include <unordered_map>
@@ -41,7 +42,8 @@ struct b2_ctx {
     uint8_t* d_bytes = nullptr; b2_run* d_runs = nullptr; uint32_t* d_run_tile_base = nullptr;
     TileRec* d_tiles = nullptr; uint32_t* d_tile_base = nullptr; uint32_t* d_tile_scratch = nullptr; uint32_t* d_tile_spec = nullptr; b2_run_status* d_run_status = nullptr;
     uint32_t* d_frame_off = nullptr; uint32_t* d_frame_run = nullptr; b2_msg_desc* d_msgs = nullptr; MsgAux* d_aux = nullptr; PackJob* d_jobs = nullptr; uint32_t* d_slow_idx = nullptr; uint8_t* d_heads = nullptr;
-    uint32_t* d_slot = nullptr; uint32_t* d_scan_tmp = nullptr; uint8_t* d_resp = nullptr; uint8_t* d_unz = nullptr; uint16_t* d_snappy_tab = nullptr; HpackState* d_hpack = nullptr; H2Conn* d_h2 = nullptr; H2Stream* d_h2_streams = nullptr; uint8_t* d_h2_slots = nullptr; uint32_t h2_max_conns = B2_H2_MAX_CONNS, h2_pending = B2_H2_MAX_PENDING, h2_stream_bytes = B2_H2_STREAM_BYTES; uint64_t h2_last_in = 0, h2_last_out = 0;   // sizes of the last h2 batch still on the device
+    uint32_t* d_slot = nullptr; uint32_t* d_scan_tmp = nullptr; uint8_t* d_resp = nullptr; uint8_t* d_unz = nullptr; uint16_t* d_snappy_tab = nullptr; HpackState* d_hpack = nullptr; H2Conn* d_h2 = nullptr; H2Stream* d_h2_streams = nullptr; uint8_t* d_h2_slots = nullptr; uint32_t h2_max_conns = B2_H2_MAX_CONNS, h2_pending = B2_H2_MAX_PENDING, h2_stream_bytes = B2_H2_STREAM_BYTES; uint64_t h2_last_in = 0, h2_last_out = 0, h2_last_unz = 0;   // sizes of the last h2 batch (and of its inflated messages) still on the device
+    uint8_t* d_h2_unz = nullptr;                                  // b2_h2_decompress_requests output (max_resp_bytes, allocated on first use)
     uint32_t* d_frame_row = nullptr; uint4* d_rows = nullptr;
     // persistent latency kernel (b2_ring_*): pinned + mapped submit ring, its own stream
     uint8_t* ring_slots = nullptr; volatile uint32_t* ring_ctl = nullptr; uint32_t* d_ring_ticket = nullptr; cudaStream_t ring_stream = nullptr;
@@ -144,7 +146,7 @@ extern "C" void b2_ctx_destroy(b2_ctx* c) {
     cudaFree(c->d_ring_ticket);
     cudaFree(c->d_bytes); cudaFree(c->d_runs); cudaFree(c->d_run_tile_base); cudaFree(c->d_tiles); cudaFree(c->d_tile_base); cudaFree(c->d_tile_scratch); cudaFree(c->d_tile_spec);
     cudaFree(c->d_run_status); cudaFree(c->d_frame_off); cudaFree(c->d_frame_run); cudaFree(c->d_msgs); cudaFree(c->d_aux); cudaFree(c->d_jobs); cudaFree(c->d_slow_idx); cudaFree(c->d_heads); cudaFree(c->d_slot);
-    cudaFree(c->d_scan_tmp); cudaFree(c->d_resp); cudaFree(c->d_unz); cudaFree(c->d_snappy_tab); cudaFree(c->d_refs); cudaFree(c->d_iov); cudaFreeHost(c->h_iov); cudaFree(c->d_frame_row); cudaFree(c->d_rows); cudaFreeHost(c->h_refs); cudaFree(c->d_hpack); cudaFree(c->d_h2); cudaFree(c->d_h2_streams); cudaFree(c->d_h2_slots); cudaFree(c->d_counters); cudaFree(c->d_totals); cudaFree(c->d_methods); cudaFree(c->d_crc_adv); cudaFree(c->d_meta); cudaFree(c->d_small); cudaFreeHost(c->h_meta); cudaFreeHost(c->h_small);
+    cudaFree(c->d_scan_tmp); cudaFree(c->d_resp); cudaFree(c->d_unz); cudaFree(c->d_snappy_tab); cudaFree(c->d_refs); cudaFree(c->d_iov); cudaFreeHost(c->h_iov); cudaFree(c->d_frame_row); cudaFree(c->d_rows); cudaFreeHost(c->h_refs); cudaFree(c->d_hpack); cudaFree(c->d_h2); cudaFree(c->d_h2_streams); cudaFree(c->d_h2_slots); cudaFree(c->d_h2_unz); cudaFree(c->d_counters); cudaFree(c->d_totals); cudaFree(c->d_methods); cudaFree(c->d_crc_adv); cudaFree(c->d_meta); cudaFree(c->d_small); cudaFreeHost(c->h_meta); cudaFreeHost(c->h_small);
     cudaFreeHost(c->h_run_status); cudaFreeHost(c->h_msgs); cudaFreeHost(c->h_resp); cudaFreeHost(c->h_totals);
     cudaFreeHost(c->h_run_tile_base);
     for (int i = 0; i <= kMaxStages; i++) if (c->ev[i]) cudaEventDestroy(c->ev[i]);
@@ -396,7 +398,7 @@ extern "C" int b2_batch_upload(b2_ctx* c, const void* bytes, uint32_t nbytes, co
             for (uint32_t t = t0; t < t1; t++) { uint32_t* q = ti + 4 * (size_t)t; q[0] = runs[r].offset; q[1] = runs[r].length; q[2] = t - t0; q[3] = r | (runs[r].flags << 24); }
         }
     }
-    c->h2_last_in = 0; c->h2_last_out = 0;       // the device copies of the last h2 batch are about to be overwritten
+    c->h2_last_in = 0; c->h2_last_out = 0; c->h2_last_unz = 0;       // the device copies of the last h2 batch are about to be overwritten
     if (c->input_mode == B2_INPUT_PULL) {
         // no copy: the kernels read the caller's pinned block in place (it must stay untouched until collect)
         void* dp = nullptr;
@@ -886,7 +888,7 @@ extern "C" int b2_crc32c_batch(b2_ctx* c, const void* bytes, uint32_t nbytes, co
     if (nbytes > c->opt.max_batch_bytes || n > c->opt.max_msgs) { set_err("exceeds ctx capacity"); return B2_E_CAPACITY; }
     for (uint32_t i = 0; i < n; i++) if ((uint64_t)offs[i] + lens[i] > nbytes) { set_err("slice outside buffer"); return B2_E_INVAL; }
     CU(cudaSetDevice(c->opt.device));
-    c->h2_last_in = 0; c->h2_last_out = 0;       // the device copies of the last h2 batch are about to be overwritten
+    c->h2_last_in = 0; c->h2_last_out = 0; c->h2_last_unz = 0;       // the device copies of the last h2 batch are about to be overwritten
     CU(cudaMemcpyAsync(c->d_bytes, bytes, nbytes, cudaMemcpyHostToDevice, c->stream));
     CU(cudaMemcpyAsync(c->d_frame_off, offs, 4 * (size_t)n, cudaMemcpyHostToDevice, c->stream));
     CU(cudaMemcpyAsync(c->d_slot, lens, 4 * (size_t)n, cudaMemcpyHostToDevice, c->stream));
@@ -930,7 +932,7 @@ extern "C" int b2_snappy_uncompress_batch(b2_ctx* c, const void* bytes, uint32_t
     CU(cudaSetDevice(c->opt.device));
     uint32_t* d_offs = c->d_frame_off; uint32_t* d_lens = c->d_slot; uint32_t* d_ooffs = c->d_frame_run;
     uint32_t* d_caps = (uint32_t*)c->d_jobs; int32_t* d_olens = (int32_t*)c->d_aux;
-    c->h2_last_in = 0; c->h2_last_out = 0;       // the device copies of the last h2 batch are about to be overwritten
+    c->h2_last_in = 0; c->h2_last_out = 0; c->h2_last_unz = 0;       // the device copies of the last h2 batch are about to be overwritten
     CU(cudaMemcpyAsync(c->d_bytes, bytes, nbytes, cudaMemcpyHostToDevice, c->stream));
     CU(cudaMemcpyAsync(d_offs, offs, 4 * (size_t)n, cudaMemcpyHostToDevice, c->stream));
     CU(cudaMemcpyAsync(d_lens, lens, 4 * (size_t)n, cudaMemcpyHostToDevice, c->stream));
@@ -967,7 +969,7 @@ extern "C" int b2_snappy_compress_batch(b2_ctx* c, const void* bytes, uint32_t n
     }
     CU(cudaSetDevice(c->opt.device));
     uint32_t* d_offs = c->d_frame_off; uint32_t* d_lens = c->d_slot; uint32_t* d_ooffs = c->d_frame_run; uint32_t* d_olens = (uint32_t*)c->d_aux;
-    c->h2_last_in = 0; c->h2_last_out = 0;       // the device copies of the last h2 batch are about to be overwritten
+    c->h2_last_in = 0; c->h2_last_out = 0; c->h2_last_unz = 0;       // the device copies of the last h2 batch are about to be overwritten
     CU(cudaMemcpyAsync(c->d_bytes, bytes, nbytes, cudaMemcpyHostToDevice, c->stream));
     CU(cudaMemcpyAsync(d_offs, offs, 4 * (size_t)n, cudaMemcpyHostToDevice, c->stream));
     CU(cudaMemcpyAsync(d_lens, lens, 4 * (size_t)n, cudaMemcpyHostToDevice, c->stream));
@@ -1073,7 +1075,7 @@ extern "C" int b2_hpack_decode_batch(b2_ctx* c, const void* bytes, uint32_t nbyt
     CU(cudaSetDevice(c->opt.device));
     uint32_t* d_conn = c->d_frame_off; uint32_t* d_off = c->d_frame_run; uint32_t* d_len = c->d_slot;
     uint32_t* d_first = (uint32_t*)c->d_jobs; uint32_t* d_olens = (uint32_t*)c->d_aux; int32_t* d_st = (int32_t*)c->d_aux + n; uint32_t* d_nh = (uint32_t*)c->d_aux + 2 * (size_t)n;
-    c->h2_last_in = 0; c->h2_last_out = 0;       // the device copies of the last h2 batch are about to be overwritten
+    c->h2_last_in = 0; c->h2_last_out = 0; c->h2_last_unz = 0;       // the device copies of the last h2 batch are about to be overwritten
     CU(cudaMemcpyAsync(c->d_bytes, bytes, nbytes, cudaMemcpyHostToDevice, c->stream));
     CU(cudaMemcpyAsync(d_conn, conn.data(), 4 * (size_t)n, cudaMemcpyHostToDevice, c->stream));
     CU(cudaMemcpyAsync(d_off, off.data(), 4 * (size_t)n, cudaMemcpyHostToDevice, c->stream));
@@ -1097,7 +1099,7 @@ extern "C" int b2_h2_scan_batch(b2_ctx* c, const void* bytes, uint32_t nbytes, c
     CU(cudaSetDevice(c->opt.device));
     static_assert(sizeof(b2_h2_frame) == sizeof(H2Frame), "frame layout");
     uint32_t* d_n = c->d_frame_off; uint32_t* d_cons = c->d_frame_run; uint32_t* d_err = c->d_slot;
-    c->h2_last_in = 0; c->h2_last_out = 0;       // the device copies of the last h2 batch are about to be overwritten
+    c->h2_last_in = 0; c->h2_last_out = 0; c->h2_last_unz = 0;       // the device copies of the last h2 batch are about to be overwritten
     CU(cudaMemcpyAsync(c->d_bytes, bytes, nbytes, cudaMemcpyHostToDevice, c->stream));
     CU(cudaMemcpyAsync(c->d_meta, runs, sizeof(b2_run) * (size_t)n_runs, cudaMemcpyHostToDevice, c->stream));
     if (n_runs) k_h2_scan<<<(n_runs + 63) / 64, 64, 0, c->stream>>>(c->d_bytes, (const b2_run*)c->d_meta, n_runs, max_frame_size, (H2Frame*)c->d_unz, cap_per_run, d_n, d_cons, d_err);
@@ -1159,7 +1161,7 @@ extern "C" int b2_h2_process_batch(b2_ctx* c, const void* bytes, uint32_t nbytes
     CU(cudaSetDevice(c->opt.device));
     b2_h2_run_status* d_rs = reinterpret_cast<b2_h2_run_status*>(c->d_run_status);      // 32 B each, like b2_run_status
     b2_h2_msg* d_msgs = reinterpret_cast<b2_h2_msg*>(c->d_msgs);                         // 64 B each, like b2_msg_desc
-    c->h2_last_in = 0; c->h2_last_out = 0;       // the device copies of the last h2 batch are about to be overwritten
+    c->h2_last_in = 0; c->h2_last_out = 0; c->h2_last_unz = 0;       // the device copies of the last h2 batch are about to be overwritten
     CU(cudaMemcpyAsync(c->d_bytes, bytes, nbytes, cudaMemcpyHostToDevice, c->stream));
     CU(cudaMemcpyAsync(c->d_meta, runs, sizeof(b2_run) * (size_t)n_runs, cudaMemcpyHostToDevice, c->stream));
     k_h2_consume<<<(n_runs + 31) / 32, 32, 0, c->stream>>>(c->d_bytes, (const b2_run*)c->d_meta, n_runs, c->d_h2, c->d_hpack, c->d_methods, c->cfg.n_methods,
@@ -1202,7 +1204,8 @@ extern "C" int b2_h2_pack_responses(b2_ctx* c, const void* bytes, uint32_t nbyte
     uint64_t total = 0;
     for (uint32_t i = 0; i < n; i++) {
         const b2_h2_response& r = resps[i];
-        const uint64_t body_lim = (r.flags & B2_H2_RESP_BODY_IN_INPUT) ? c->h2_last_in : (r.flags & B2_H2_RESP_BODY_IN_OUT) ? c->h2_last_out : nbytes;
+        const uint64_t body_lim = (r.flags & B2_H2_RESP_BODY_IN_INPUT) ? c->h2_last_in : (r.flags & B2_H2_RESP_BODY_IN_OUT) ? c->h2_last_out :
+                                  (r.flags & B2_H2_RESP_BODY_IN_UNZ) ? c->h2_last_unz : nbytes;
         const uint64_t ct_lim = (r.flags & B2_H2_RESP_CT_IN_OUT) ? c->h2_last_out : nbytes;
         if (r.conn >= c->h2_max_conns || (uint64_t)r.body_off + r.body_len > body_lim || (uint64_t)r.content_type_off + r.content_type_len > ct_lim ||
             (uint64_t)r.grpc_message_off + r.grpc_message_len > nbytes || r.content_type_len > 256 || r.grpc_message_len > 512) { set_err("bad response descriptor"); return B2_E_INVAL; }
@@ -1227,11 +1230,58 @@ extern "C" int b2_h2_pack_responses(b2_ctx* c, const void* bytes, uint32_t nbyte
     CU(cudaMemcpyAsync(d_resps, resps, sizeof(b2_h2_response) * (size_t)n, cudaMemcpyHostToDevice, c->stream));
     CU(cudaMemcpyAsync(d_first, first.data(), 4 * first.size(), cudaMemcpyHostToDevice, c->stream));
     CU(cudaMemcpyAsync(d_offs, out_offs, 4 * (size_t)n, cudaMemcpyHostToDevice, c->stream));
-    k_h2_pack<<<(n_groups + kH2PackWarps - 1) / kH2PackWarps, kH2PackWarps * 32, 0, c->stream>>>(d_aux, c->d_bytes, c->d_unz, d_resps, d_first, n_groups, c->d_h2, c->d_resp, d_offs, d_lens);
+    k_h2_pack<<<(n_groups + kH2PackWarps - 1) / kH2PackWarps, kH2PackWarps * 32, 0, c->stream>>>(d_aux, c->d_bytes, c->d_unz, c->d_h2_unz, d_resps, d_first, n_groups, c->d_h2, c->d_resp, d_offs, d_lens);
     CU(cudaMemcpyAsync(out_lens, d_lens, 4 * (size_t)n, cudaMemcpyDeviceToHost, c->stream));
     CU(cudaMemcpyAsync(out, c->d_resp, (size_t)total, cudaMemcpyDeviceToHost, c->stream));
     CU(cudaStreamSynchronize(c->stream));
     c->uploaded = false; c->executed = false;
+    return B2_OK;
+}
+
+// GzipDecompress of ProcessHttpRequest over messages of the last h2 batch: see include/b2rpc.h
+extern "C" int b2_h2_decompress_requests(b2_ctx* c, const b2_h2_msg* msgs, uint32_t n, void* out, uint32_t out_cap, b2_h2_unz_result* res) {
+    if (!c || (n && (!msgs || !res)) || (!out && out_cap)) { set_err("null argument"); return B2_E_INVAL; }
+    static_assert(sizeof(b2_h2_unz_result) == 16, "h2 unz ABI layout");
+    if (c->h2_last_out == 0) { set_err("no h2 batch is live on this context"); return B2_E_INVAL; }
+    if (n > c->opt.max_msgs || out_cap > c->opt.max_resp_bytes) { set_err("exceeds ctx capacity"); return B2_E_CAPACITY; }
+    for (uint32_t i = 0; i < n; i++) {         // descriptors come from the caller: every range inside the buffers of the live batch
+        const b2_h2_msg& m = msgs[i];
+        const uint64_t lim = (m.flags & B2_H2_FLAG_BODY_IN_INPUT) ? c->h2_last_in : c->h2_last_out;
+        const uint64_t out_end = std::max<uint64_t>((uint64_t)m.headers_off + m.headers_len, (m.flags & B2_H2_FLAG_BODY_IN_INPUT) ? 0 :
+                                                    std::max<uint64_t>((uint64_t)m.body_off + m.body_len, (uint64_t)m.msg_off + m.msg_len));
+        if ((uint64_t)m.headers_off + m.headers_len > c->h2_last_out || (uint64_t)m.body_off + m.body_len > lim || (uint64_t)m.msg_off + m.msg_len > lim) {
+            set_err("a message lies outside the last h2 batch"); return B2_E_INVAL;
+        }
+        // b2_h2_pack_responses stages its bytes in the second half of the scratch: only the first max_resp_bytes of the out buffer stay
+        if (out_end > c->opt.max_resp_bytes) { set_err("last h2 out buffer too large to stay resident"); return B2_E_CAPACITY; }
+    }
+    c->h2_last_unz = 0;
+    if (n == 0) return B2_OK;
+    CU(cudaSetDevice(c->opt.device));
+    if (!c->d_h2_unz) CU(cudaMalloc(&c->d_h2_unz, (size_t)c->opt.max_resp_bytes + 16));
+    b2_h2_msg* d_msgs = reinterpret_cast<b2_h2_msg*>(c->d_msgs);                 // the batch's own descriptors were fetched by b2_h2_process_batch
+    b2_h2_unz_result* d_res = reinterpret_cast<b2_h2_unz_result*>(c->d_aux);      // 16 B <= sizeof(MsgAux) per message
+    static_assert(sizeof(MsgAux) >= sizeof(b2_h2_unz_result), "unz results live in the aux array");
+    CU(cudaMemcpyAsync(d_msgs, msgs, sizeof(b2_h2_msg) * (size_t)n, cudaMemcpyHostToDevice, c->stream));
+    const uint32_t grid = (n + kH2UnzWarps - 1) / kH2UnzWarps;
+    c->stage_names[0] = "h2_inflate_size"; c->stage_names[1] = "h2_unz_offsets"; c->stage_names[2] = "h2_inflate_write";
+    CU(cudaEventRecord(c->ev[0], c->stream));
+    k_h2_inflate<false><<<grid, kH2UnzWarps * 32, 0, c->stream>>>(c->d_bytes, c->d_unz, d_msgs, n, d_res, c->d_h2_unz);
+    CU(cudaEventRecord(c->ev[1], c->stream));
+    k_h2_unz_offsets<<<1, kUnzScanBlock, 0, c->stream>>>(d_res, n, out_cap);
+    CU(cudaEventRecord(c->ev[2], c->stream));
+    k_h2_inflate<true><<<grid, kH2UnzWarps * 32, 0, c->stream>>>(c->d_bytes, c->d_unz, d_msgs, n, d_res, c->d_h2_unz);
+    CU(cudaEventRecord(c->ev[3], c->stream));
+    c->n_stages = 3;
+    CU(cudaMemcpyAsync(res, d_res, sizeof(b2_h2_unz_result) * (size_t)n, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    uint64_t end = 0;                                                             // only the bytes produced go back
+    for (uint32_t i = 0; i < n; i++) if (res[i].status == B2_H2_UNZ_OK) end = std::max<uint64_t>(end, (uint64_t)res[i].out_off + res[i].out_len);
+    if (end) {
+        CU(cudaMemcpyAsync(out, c->d_h2_unz, (size_t)end, cudaMemcpyDeviceToHost, c->stream));
+        CU(cudaStreamSynchronize(c->stream));
+    }
+    c->h2_last_unz = end;
     return B2_OK;
 }
 
@@ -1332,7 +1382,7 @@ extern "C" int b2_pack_requests(b2_ctx* c, const void* bytes, uint32_t nbytes, c
     CU(cudaSetDevice(c->opt.device));
     ReqDesc* d_reqs = reinterpret_cast<ReqDesc*>(c->d_msgs);
     uint32_t* d_offs = c->d_frame_off; uint32_t* d_lens = c->d_slot;
-    c->h2_last_in = 0; c->h2_last_out = 0;       // the device copies of the last h2 batch are about to be overwritten
+    c->h2_last_in = 0; c->h2_last_out = 0; c->h2_last_unz = 0;       // the device copies of the last h2 batch are about to be overwritten
     if (nbytes) CU(cudaMemcpyAsync(c->d_bytes, bytes, nbytes, cudaMemcpyHostToDevice, c->stream));
     CU(cudaMemcpyAsync(d_reqs, reqs, sizeof(b2_request) * (size_t)n, cudaMemcpyHostToDevice, c->stream));
     CU(cudaMemcpyAsync(d_offs, out_offs, 4 * (size_t)n, cudaMemcpyHostToDevice, c->stream));
@@ -1373,7 +1423,7 @@ extern "C" int b2_pack_responses(b2_ctx* c, const void* bytes, uint32_t nbytes, 
     CU(cudaSetDevice(c->opt.device));
     ReplyDesc* d_reps = reinterpret_cast<ReplyDesc*>(c->d_msgs);
     uint32_t* d_offs = c->d_frame_off; uint32_t* d_lens = c->d_slot;
-    c->h2_last_in = 0; c->h2_last_out = 0;
+    c->h2_last_in = 0; c->h2_last_out = 0; c->h2_last_unz = 0;
     if (nbytes) CU(cudaMemcpyAsync(c->d_bytes, bytes, nbytes, cudaMemcpyHostToDevice, c->stream));
     CU(cudaMemcpyAsync(d_reps, reps, sizeof(b2_reply) * (size_t)n, cudaMemcpyHostToDevice, c->stream));
     CU(cudaMemcpyAsync(d_offs, out_offs, 4 * (size_t)n, cudaMemcpyHostToDevice, c->stream));

@@ -2857,5 +2857,32 @@ __global__ void __launch_bounds__(kSmallThreads, 1) k_ring(RingDev R, BatchPtrs 
     if (tid == 0) *R.next_ticket = ticket;
 }
 
+// b2_h2_decompress_requests: the output slots of the messages to inflate (B2_H2_UNZ_OK, out_len = the sizing bound), back to back in
+// message order: an exclusive scan of the bounds by one block, each thread a contiguous run of messages.  A message whose slot would
+// end past out_cap is B2_H2_UNZ_NO_ROOM, and so is every later one with a non-empty bound (the running sum keeps its bound).
+constexpr uint32_t kUnzScanBlock = 1024;
+__global__ void __launch_bounds__(kUnzScanBlock) k_h2_unz_offsets(b2_h2_unz_result* res, uint32_t n, uint32_t out_cap) {
+    __shared__ unsigned long long s[kUnzScanBlock];
+    const uint32_t t = threadIdx.x, per = (n + kUnzScanBlock - 1) / kUnzScanBlock, b = min(t * per, n), e = min(b + per, n);
+    unsigned long long sum = 0;
+    for (uint32_t i = b; i < e; i++) if (res[i].status == B2_H2_UNZ_OK) sum += res[i].out_len;
+    s[t] = sum;
+    __syncthreads();
+    for (uint32_t d = 1; d < kUnzScanBlock; d <<= 1) {
+        const unsigned long long v = t >= d ? s[t - d] : 0ull;
+        __syncthreads();
+        s[t] += v;
+        __syncthreads();
+    }
+    unsigned long long off = s[t] - sum;
+    for (uint32_t i = b; i < e; i++) {
+        if (res[i].status != B2_H2_UNZ_OK) continue;
+        const uint32_t bound = res[i].out_len;
+        if (off + bound > out_cap) { res[i].status = B2_H2_UNZ_NO_ROOM; res[i].out_len = 0; }
+        else res[i].out_off = (uint32_t)off;
+        off += bound;
+    }
+}
+
 #endif  // __CUDACC__
 }  // namespace b2

@@ -375,7 +375,7 @@ int  b2_batch_info(b2_ctx* ctx, uint32_t out[4]);
  * their rate.  No ctx needed.  (brpc pins nothing itself; its RDMA endpoint leaves NUMA placement to the deployment as well.) */
 int  b2_device_pci_bus_id(int device, char* out, int cap);
 
-/* Device time of each stage of the last execute, in launch order.  Writes up to
+/* Device time of each stage of the last execute (or b2_h2_decompress_requests), in launch order.  Writes up to
  * `cap` entries of (name, ms); returns the number of stages. */
 int  b2_stage_times(b2_ctx* ctx, const char** names, float* ms, int cap);
 
@@ -572,6 +572,7 @@ int  b2_h2_process_batch(b2_ctx* ctx, const void* bytes, uint32_t nbytes, const 
 #define B2_H2_RESP_BODY_IN_INPUT 2u   /* body_off indexes that call's input bytes (e.g. an echoed B2_H2_FLAG_BODY_IN_INPUT message) */
 #define B2_H2_RESP_BODY_IN_OUT   4u   /* body_off indexes that call's out buffer */
 #define B2_H2_RESP_CT_IN_OUT     8u   /* content_type_off indexes that call's out buffer (the request's own content-type value) */
+#define B2_H2_RESP_BODY_IN_UNZ  16u   /* body_off indexes the last b2_h2_decompress_requests output (zero copy) */
 typedef struct b2_h2_response {
     uint32_t conn, stream_id;
     int32_t  status_code;                            /* :status */
@@ -584,6 +585,32 @@ typedef struct b2_h2_response {
 } b2_h2_response;                                    /* 48 bytes */
 int  b2_h2_pack_responses(b2_ctx* ctx, const void* bytes, uint32_t nbytes, const b2_h2_response* resps, uint32_t n,
                           void* out, uint32_t out_cap, uint32_t* out_offs, uint32_t* out_lens);
+
+/* b2_h2_decompress_requests: the GzipDecompress step of ProcessHttpRequest (src/brpc/policy/http_rpc_protocol.cpp:1646-1683) for
+ * messages of the LAST b2_h2_process_batch on this context (their header records and bodies are still on the device).
+ *   - gRPC (B2_H2_FLAG_GRPC): only a message whose prefix is valid (B2_H2_FLAG_GRPC_PREFIX_OK) and has the compressed flag is looked
+ *     at; its encoding is the "grpc-encoding" header, and a missing header is the reference's EREQUEST "Fail to find header
+ *     `grpc-encoding' in compressed gRPC request".  The message (msg_off/msg_len) is inflated.
+ *   - otherwise a non-empty body's encoding is the "content-encoding" header, and the whole body is inflated.
+ *   - headers are looked up the way HttpHeader keeps them (http_header.cpp:100-116): names case-insensitively, a repeated header
+ *     folded with "," onto a non-empty value (an empty value is overwritten).  Only the exact value "gzip" is inflated
+ *     (policy::GzipDecompress, gzip_compress.cpp:138-176,187-190); any other value leaves the bytes to the parser as they are.
+ * Messages are taken in the order given and the caller passes the ones it would parse (method_idx is not looked at).  Inflated
+ * messages are laid out back to back in `out` in message order; a message that does not fit into out_cap after the earlier ones
+ * is B2_H2_UNZ_NO_ROOM.  Only the bytes up to the end of the last inflated message are written.  The output also stays on the
+ * device for b2_h2_pack_responses (B2_H2_RESP_BODY_IN_UNZ) as long as the batch does (the rule of B2_H2_RESP_BODY_IN_INPUT).
+ * Replies are not compressed (brpc compresses one only when the service sets response_compress_type, :971-994).
+ * out_cap <= max_resp_bytes.  B2_E_INVAL: no h2 batch is live, or a message's ranges lie outside that batch's buffers. */
+#define B2_H2_UNZ_NONE        0   /* nothing to inflate (not compressed / not gzip-encoded body): the message is msg_off/msg_len, or the body */
+#define B2_H2_UNZ_OK          1   /* inflated: out[out_off, +out_len) */
+#define B2_H2_UNZ_NO_ENCODING 2   /* compressed gRPC message, no grpc-encoding header -> EREQUEST (text above) */
+#define B2_H2_UNZ_NOT_GZIP    3   /* compressed / encoded, but the (folded) value is not "gzip": parsed as it is */
+#define B2_H2_UNZ_FAILED      4   /* GzipDecompress returned false -> EREQUEST "Fail to un-gzip request body" (a body in one block
+                                     never yields it: DESIGN §5) */
+#define B2_H2_UNZ_HOST        5   /* input or output beyond 1 MiB: left to the host, like B2_MSG_UNSUPPORTED */
+#define B2_H2_UNZ_NO_ROOM     6   /* out_cap used up by earlier messages of this call */
+typedef struct b2_h2_unz_result { uint32_t status, out_off, out_len, reserved; } b2_h2_unz_result;   /* 16 bytes */
+int  b2_h2_decompress_requests(b2_ctx* ctx, const b2_h2_msg* msgs, uint32_t n, void* out, uint32_t out_cap, b2_h2_unz_result* res);
 
 /* b2_h2_pack_requests — the CLIENT side of the same connection state: H2UnsentRequest::New (src/brpc/policy/http2_rpc_protocol.cpp:
  * 1382-1453: the header list) + H2UnsentRequest::AppendAndDestroySelf (:1496-1592) + PackH2Message (:1310-1380), what PackH2Request
